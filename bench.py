@@ -1,7 +1,11 @@
 #!/usr/bin/env python
 """bench.py — Mrays/s of the NeRFshop render path at 1920x1080 on the synthetic nerf/fox-shaped workload.
 
-  python bench.py --gpus N --steps K --warmup W [--impl native|reference]
+  python bench.py --gpus N --steps K --warmup W [--impl native|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step computed, as a caller of the render path receives it, to DIR/rgba.npy
+([1080, 1920, 4] float32) and DIR/depth.npy ([1080, 1920] float32). The inputs depend on the arguments only (seeded parameters,
+camera index 7*step mod 120), so two builds run with the same arguments can be compared output for output.
 
 A "step" is one frame: Testbed::render_nerf of one camera of a 120-view orbit (a different camera every
 step = free-viewpoint orbit), base.json network (hash L=16 F=2 T=2^19, MLPs 64x1 / 64x2), synthetic seeded
@@ -270,7 +274,10 @@ def main():
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-baseline", action="store_true", help="skip the reference-CUDA arm and the edit configurations (N = 1 extras)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's RGBA and depth as DIR/rgba.npy and DIR/depth.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to --impl native")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world == 1:
@@ -295,8 +302,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps = max(1, min(args.steps, 8))
-        warm = max(3, min(args.warmup, 3))
+        steps, warm = args.steps, args.warmup
         mrays, ms, cores, spf, kind, (p10, p90) = cpu_reference_run(steps, warm)
         sample = f"{CPU_W}x{CPU_H} frame (1/64 of the 1080p pixels) of the same orbit per step, {cores} pinned threads, median of {steps} steps (p10 {p10:.0f} ms, p90 {p90:.0f} ms), {warm} warm-up"
         note = ("the reference's Testbed::render_nerf / NerfTracer::trace / kernels compiled for the CPU from /root/reference (oracle/_ref); tiny-cuda-nn's network (absent submodule) = the oracle's CPU restatement"
@@ -385,6 +391,10 @@ def main():
         sampler.start()
     total_ms, wall, kern_ms, samples = timed(device_step, args.warmup, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # fb / depth still hold the last timed step (for N > 1: the gathered frame)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "rgba.npy"), fb.cpu().numpy())
+        np.save(os.path.join(args.dump_outputs, "depth.npy"), depth.cpu().numpy())
 
     # ---- e2e: every step's frame ends in (pinned) HOST memory; the copy of frame k overlaps the render of frame k+1, two frames in flight ----
     # N = 1: the C ABI's host-buffer entry point nsb_render_host_async / nsb_host_frame_wait (the consumer takes frame k-1 while frame k renders).

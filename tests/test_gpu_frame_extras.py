@@ -9,8 +9,10 @@ import pytest
 
 from nerfshop_b200 import abi
 from nerfshop_b200 import synthetic as syn
-from oracle import ref, ref_build
+from ref_golden import Recorded
 from test_frame_extras_cpu import CASES, H, W, _dof
+
+ref = Recorded("gpu_frame_extras")  # outputs of oracle/_ref's CUDA build stored under tests/golden/ref/ (ref_golden.py)
 
 pytestmark = pytest.mark.gpu
 
@@ -58,7 +60,6 @@ def test_native_vs_oracle(scene, oracle, renderer, maps, case):
     assert np.abs(depth - d_o)[hit].max() < 0.25
 
 
-@pytest.mark.skipif(ref_build.build_cuda() is None, reason="oracle/_ref CUDA library not built and /root/reference absent")
 @pytest.mark.parametrize("case", list(CASES))
 def test_native_vs_reference_cuda(scene, renderer, maps, case):
     import torch
@@ -68,14 +69,18 @@ def test_native_vs_reference_cuda(scene, renderer, maps, case):
     try:
         _, f_dev = _frames(model, case, maps, cam=63, w=320, h=180)
         fb, depth = renderer.render(f_dev)
-        fb_r, depth_r, info = rc.render(f_dev, renderer)
+        # the reference's frame is stored at a seeded sample of 12,000 of the 57,600 pixels
+        sel = torch.from_numpy(np.sort(np.random.default_rng(11).choice(320 * 180, 12_000, replace=False))).cuda()
+        fb_r, depth_r, info = rc.render(f_dev, renderer, shrink=lambda o: (o[0].reshape(-1, 4)[sel], None, o[2]), also=(maps["env"], maps["dist"]))
         torch.cuda.synchronize()
+        fb = fb.reshape(-1, 4)[sel]
         err = ((fb - fb_r).abs() / fb_r.abs().clamp(min=1.0)).amax(-1)
         n_bad = int((err > 1e-3).sum())
         print(f"\n{case}: native vs the reference's CUDA path L-inf {float(err.max()):.3e}; pixels > 1e-4: {int((err > 1e-4).sum())} of {err.numel()}; identical: {bool(torch.equal(fb, fb_r))}")
         assert (fb_r[..., 3] > 0).float().mean().item() > 0.2
-        # termination flips are not masked here (no margin from the reference): allow a handful of pixels
-        assert n_bad <= 6 and float(err.max()) < 5e-2
+        # termination flips are not masked here (no margin from the reference): allow a handful of pixels, 6 in the whole frame,
+        # at that rate over the sample
+        assert n_bad <= int(np.ceil(6 * sel.numel() / (320 * 180))) and float(err.max()) < 5e-2
         assert float((err > 1e-4).float().mean()) < 0.02
     finally:
         rc.close()
